@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — interpolated frames/s of the GIMM-VFI-R per-pair path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = one GIMMVFI_R.forward over one batch of synthetic frame pairs.  Workload at
 every N: BASELINE.json configs[1] — one 1920x1080 pair per GPU (caller-padded to
@@ -27,6 +27,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 METRIC = "interpolated frames/sec @1080p t=0.5"
@@ -85,6 +86,35 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(self.rows)}
 
 
+DUMP_BUDGET = 60 << 20   # bytes of array data --dump-outputs writes at most (the .npy headers stay well inside 64 MB)
+
+
+def flatten_outputs(out, prefix=""):
+    """{name: tensor} of a forward's output dict; list entries append their index (imgt_pred_0, flowt0_pred_0_1, ...)"""
+    if torch.is_tensor(out):
+        return {prefix: out}
+    items = {}
+    for k, v in (out.items() if isinstance(out, dict) else enumerate(out)):
+        items.update(flatten_outputs(v, "%s_%s" % (prefix, k) if prefix else str(k)))
+    return items
+
+
+def dump_outputs(path, out):
+    """Writes every array of `out` as <path>/<name>.npy in float32 (float64 stays float64).  If they exceed DUMP_BUDGET together,
+    each array larger than an equal share of it is replaced by a 1-D sample of that many elements: flat indices drawn without
+    replacement by numpy.random.default_rng(0), in increasing order, so runs of two builds write the same elements."""
+    arrays = flatten_outputs(out)
+    os.makedirs(path, exist_ok=True)
+    total = sum(t.numel() * (8 if t.dtype == torch.float64 else 4) for t in arrays.values())
+    share = DUMP_BUDGET // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().to("cpu", torch.float64 if t.dtype == torch.float64 else torch.float32).numpy()
+        cap = share // a.itemsize
+        if total > DUMP_BUDGET and a.size > cap:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def cpu_threads():
     """Threads for the CPU arm: all host cores up to GIMMVFI_CPU_THREADS (default 64: the builder's 1080p run, 104.5 s per frame,
     used 64 of the GPU box's 128 cores; the reference's small RAFT convolutions oversubscribe oneDNN beyond that)."""
@@ -118,18 +148,18 @@ def cpu_reference_fps(steps, warmup, H=H_PAD, W=W_PAD, T=1):
     with torch.no_grad():
         for i in range(warmup + steps):
             t0 = time.perf_counter()
-            O.gimmvfi_r_forward(sd, xs, coord, t)
+            out = O.gimmvfi_r_forward(sd, xs, coord, t)
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
     sec = sum(times) / len(times)
-    return dict(sec_per_step=sec, fps=T / sec, cores=torch.get_num_threads(), times=times)
+    return dict(sec_per_step=sec, fps=T / sec, cores=torch.get_num_threads(), times=times, out=out)
 
 
 def run_reference(args, rank):
     """--impl reference: the reference's CPU implementation of the SAME config (one 1088x1920 pair per step).  A forward takes
-    ~100 s on the box's host cores, so the number of forwards actually run is bounded (GIMMVFI_REF_MAX_STEPS timed, default 2, after
-    at most one warm-up) — `steps`/`warmup` echo the request, `steps_timed`/`warmup_run` say what ran."""
+    ~100 s on the box's host cores, so the warm-up is bounded (at most GIMMVFI_REF_MAX_WARMUP forwards, default 1); --steps
+    forwards are timed.  `steps`/`warmup` echo the request, `steps_timed`/`warmup_run` say what ran."""
     if rank != 0:
         return
     H, W = args.height, args.width
@@ -138,12 +168,14 @@ def run_reference(args, rank):
         H, W = (int(v) for v in os.environ["GIMMVFI_CPU_SAMPLE"].lower().split("x"))
         scaled = (H * W) / float(args.height * args.width)
     T = max(1, args.timesteps)
-    timed = max(1, min(args.steps, int(os.environ.get("GIMMVFI_REF_MAX_STEPS", "2"))))
+    timed = args.steps
     warm = min(max(0, args.warmup), int(os.environ.get("GIMMVFI_REF_MAX_WARMUP", "1")))
     r = cpu_reference_fps(timed, warm, H, W, T)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["out"])
     fps = r["fps"] * (scaled if scaled else 1.0)
     sample = ("oracle port (== reference PyTorch fp32 path, bit-identical to it on the golden fixtures) on the full %dx%d pair, "
-              "%d warm-up + %d timed forwards of %d requested (bounded: ~100 s each)" % (H, W, warm, timed, args.steps))
+              "%d warm-up + %d timed forwards (~100 s each)" % (H, W, warm, timed))
     if scaled:
         sample = "TEST SAMPLE %dx%d pixel-scaled to %dx%d — not the benchmark config" % (H, W, args.height, args.width)
     cfg = workload_config(args.height, args.width, T)
@@ -279,7 +311,12 @@ def main():
     ap.add_argument("--profile-json", default="", help="write the per-kernel CUDA-event breakdown here")
     ap.add_argument("--timesteps", type=int, default=1,
                     help="T interpolated frames per pair at t = i/(T+1): 1 = the headline metric (t=0.5); 7 = the reference's N=8 video setting")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32; at most 64 MB in all, larger "
+                         "outputs as a fixed seeded sample of their elements) - the inputs are seeded, so runs of two builds compare output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     batch_mode = args.config == "batch720"
     f_mode = args.config in ("f2k", "f4k")
     ds = None
@@ -355,12 +392,14 @@ def main():
         return (torch.stack(out["imgt_pred"], 1).reshape(-1, 3, H, W) if T > 1 else out["imgt_pred"][0])[: b * T]
 
     def step(x=None):
-        """one step on device-resident inputs: pair1080 = one forward; batch720 = this rank's shard in micro-batches + ONE all-gather"""
+        """one step on device-resident inputs: pair1080 = one forward; batch720 = this rank's shard in micro-batches + ONE all-gather.
+        Returns what the caller receives: the forward's output dict, or this rank's frames (batch720)."""
         if not batch_mode:
-            img = frames_of(model(xs if x is None else x, coord, t=tt, **fkw), B)
+            out = model(xs if x is None else x, coord, t=tt, **fkw)
+            img = frames_of(out, B)
             if world > 1:
                 dist.all_gather_into_tensor(gathered, img.contiguous())   # the single output collective
-            return img
+            return out
         done = 0
         for m in range(nmb):
             b = min(MB, len(mine) - done)
@@ -368,7 +407,7 @@ def main():
             done += b
         if world > 1:
             dist.all_gather_into_tensor(gathered, outbuf)
-        return outbuf
+        return {"imgt_pred": outbuf}
 
     def barrier():
         if world > 1:
@@ -389,14 +428,18 @@ def main():
     barrier()
     wall0 = time.perf_counter()
     for _ in range(args.steps):
+        last = None   # a step's outputs are released before the next step starts
         flush.fill_(1)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        step()
+        last = step()
         e1.record()
         evs.append((e0, e1))
     barrier()
     wall = time.perf_counter() - wall0
+    if args.dump_outputs and rank == 0:   # written after the measurements below
+        dumped = {k: v.cpu() for k, v in flatten_outputs(last).items()}
+    del last
     ms = sum(a.elapsed_time(b) for a, b in evs) / args.steps
     launches = model.engine.last_launches * nmb
     # ---- end-to-end through the public API: pinned host input -> H2D -> forward -> D2H of the frames, every forward.
@@ -548,6 +591,8 @@ def main():
                 line["cpu_baseline"] = cb
             except Exception as ex:  # noqa: BLE001
                 line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": cpu_threads(), "kind": "port", "sample": "CPU arm did not finish within 240 s: %r" % (ex,)}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

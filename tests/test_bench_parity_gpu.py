@@ -10,12 +10,15 @@ Contract (BASELINE.json north_star): max |d imgt_pred| <= 1e-3 in the DEFAULT pr
 grid; additionally the PSNR-equivalent (RMSE) and the flow fields' percentiles are bounded as in test_forward_gpu.py."""
 import json
 import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
 
+import gimmvfi_r_oracle as O
 from conftest import GOLDEN_DIR
 from gimmvfi_b200 import GIMMVFI_R
 from gimmvfi_b200.synth import synth_batch
@@ -82,3 +85,26 @@ def test_benchmarked_config_matches_reference(name, model):
     report = "; ".join("%s %.3e (<= %.1e)%s" % (n, v, lim, "" if v <= lim else " FAIL") for n, v, lim in checks)
     print(name, "mode", model.tensor_cores, report)
     assert all(v <= lim for _, v, lim in checks), report
+
+
+def test_bench_dump_outputs_hold_the_timed_forward(tmp_path, weights0):
+    """bench.py --dump-outputs on the GPU path: the files hold the last timed forward's outputs on the seeded input (synth seed 100,
+    weights seed 0) - imgt_pred within the parity tolerance of the CPU oracle on the same input."""
+    H, W = 128, 160
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--height", str(H), "--width", str(W), "--steps", "2", "--warmup", "1",
+                        "--no-cpu-baseline", "--no-torch-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=root)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+    assert d["steps"] == 2 and d["config"]["height"] == H and d["config"]["width"] == W
+    names = sorted(p.name for p in tmp_path.iterdir())
+    assert {"imgt_pred_0.npy", "flowt_0.npy", "raft_flow.npy", "nflow.npy"} <= set(names), names
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 << 20
+    assert all(np.load(tmp_path / n).dtype == np.float32 for n in names)
+    with torch.no_grad():
+        ref = O.gimmvfi_r_forward(weights0, synth_batch(1, H, W, seed=100), [(O.sample_coord_input(1, (H, W), [0.5]), None)], [0.5 * torch.ones(1)])
+    img = np.load(tmp_path / "imgt_pred_0.npy")
+    assert img.shape == (1, 3, H, W)
+    err = np.abs(img - ref["imgt_pred"][0].numpy()).max()
+    print("bench dump: imgt_pred max|d| vs oracle = %.3e" % err)
+    assert err <= TOL_IMG, err
